@@ -1,17 +1,17 @@
 """GPU results against the REFERENCE'S OWN planner sources directly (oracle/_ref/libmplref.so, see oracle/ref_harness.cpp),
-without the oracle in between.  The library is built where /root/reference exists and travels to the GPU box with the
-snapshot; the tests skip when it is absent."""
+without the oracle in between.  The reference side replays tests/golden/reference_calls/test_gpu_vs_reference.npz (see
+tests/ref_replay.py)."""
 import numpy as np
 import pytest
 
 import oracle
-from oracle import ref
+import ref_replay as ref
+from ref_replay import recorded_reference  # noqa: F401 (autouse fixture)
 import mpl_ros_b200 as mp
 from mpl_ros_b200 import maps
 from helpers import load_config
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not ref.available(), reason="oracle/_ref/libmplref.so not present")]
+pytestmark = pytest.mark.gpu
 
 FIELDS = ("n_seg", "cost", "pops", "n_nodes", "n_open", "n_closed", "n_prims", "n_valid", "pop_hash", "closed_hash")
 
@@ -71,7 +71,7 @@ def test_single_plans(name):
     if name == "corridor":
         assert rr["n_closed"] == 615 and rr["cost"] == 351.5  # MPL/README.md:200-202 out of the reference's own code
     gn = pl.getNodes()
-    assert np.array_equal(gn["key"][pl.getPopLog()], rp.pop_keys(rr["pops"]))
+    assert ref.same(gn["key"][pl.getPopLog()], rp.pop_keys(rr["pops"]))
     # trajectory: coefficient rows of every primitive (what toTrajectoryROSMsg would publish)
     coeffs = rp.traj_coeffs(rr["n_seg"])
     prs = pl.getTraj().getPrimitives()
@@ -115,9 +115,9 @@ def test_cost_shaping_flow():
     rp.set_vec("potential_radius", [1.0, 1.0, 0.0])
     pl.updatePotentialMap(start)
     rp.update_potential_map(np.array([start[0], start[1], 0.0]))
-    assert np.array_equal(pl._keep.getMap(), rp._keep.get_data())
+    assert ref.same(pl._keep.getMap(), rp._keep.get_data())
     pl.plan(sg, gg)
     rr = rp.plan(sr, gr)
     _same(pl.result(), rr, "shaped")
     gn = pl.getNodes()
-    assert np.array_equal(gn["key"][pl.getPopLog()], rp.pop_keys(rr["pops"]))
+    assert ref.same(gn["key"][pl.getPopLog()], rp.pop_keys(rr["pops"]))

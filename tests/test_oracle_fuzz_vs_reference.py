@@ -2,15 +2,15 @@
 oracle/ref_harness.cpp): random 2D / 3D box maps, controls (VEL / ACC / JRK / SNP and the yaw variants), control sets,
 bounds, dt, w, epsilon, tolerances, max_num, start velocities, unknown cells, potential maps with local ranges and
 search regions along random paths.  Every counter and both key hashes must agree exactly.  (An offline run of the same
-generators over 500 cases found no mismatch; the test keeps 64.)  Skipped where the library is absent."""
+generators over 500 cases found no mismatch; the test keeps 64.)  The reference side replays
+tests/golden/reference_calls/test_oracle_fuzz_vs_reference.npz (see tests/ref_replay.py)."""
 import numpy as np
 import pytest
 
 import oracle
-from oracle import ref
+import ref_replay as ref
+from ref_replay import recorded_reference  # noqa: F401 (autouse fixture)
 from mpl_ros_b200 import maps
-
-pytestmark = pytest.mark.skipif(not ref.available(), reason="oracle/_ref/libmplref.so not built (needs /root/reference)")
 
 FIELDS=("cost","pops","n_nodes","n_open","n_closed","n_prims","n_valid","pop_hash","closed_hash")
 def rand_case(rng, dim):
@@ -99,7 +99,7 @@ def run_shaped(seed, dim):
             p.set_vec("potential_radius", pr); p.set_vec("potential_map_range", rngv)
             p.update_potential_map(np.r_[start, np.zeros(3-dim)])
         ncell=int(np.prod(nd))
-        if not np.array_equal(om.get_data(ncell), rm.get_data()): extra.append("potmap")
+        if not ref.same(om.get_data(ncell), rm.get_data()): extra.append("potmap")
         if rng.random() < 0.6:
             npts = rng.integers(2, 6)
             path = np.zeros((npts,3)); path[0,:dim]=start; path[-1,:dim]=goal

@@ -1,5 +1,6 @@
 """LPA* (SURVEY 8f.3) on the CPU side of the parity chain:
-(1) the oracle's literal restatement equals the reference's OWN LPA* sources (oracle/_ref, skipped where absent) step by step
+(1) the oracle's literal restatement equals the reference's OWN LPA* sources (oracle/_ref, replayed from
+    tests/golden/reference_calls/, see tests/ref_replay.py) step by step
     over the replanning flows of tests/lpa_flow.py — result records, the whole state space in hm_ order (key, g, rhs, h,
     flags, hashes of the stored successor / predecessor lists), the priority-queue ARRAY, best_child_, the linked points;
 (2) the oracle reproduces the committed fixture recorded from those sources (tests/golden/lpa_flows.npz);
@@ -14,7 +15,8 @@ import numpy as np
 import pytest
 
 import oracle
-from oracle import ref
+import ref_replay as ref
+from ref_replay import recorded_reference  # noqa: F401 (autouse fixture)
 import lpa_emul
 import lpa_flow
 
@@ -22,7 +24,6 @@ GOLD = os.path.join(os.path.dirname(__file__), "golden", "lpa_flows.npz")
 FAST = [n for n in lpa_flow.FLOWS if n != "skir_jrk"]
 
 
-@pytest.mark.skipif(not ref.available(), reason="needs oracle/_ref (built from /root/reference)")
 @pytest.mark.parametrize("name", FAST)
 def test_oracle_equals_reference_sources(name):
     a, _ = lpa_flow.run_flow(name, ref.RefMap, ref.RefPlanner)

@@ -1,8 +1,8 @@
 """Seeded random LPA* replanning sequences: random 2D / 3D box maps, controls (VEL / ACC / JRK / SNP), control sets, bounds,
 epsilon, max_num; then rounds of { drop a random patch of obstacle cells near the trajectory | clear some of the cells dropped
 earlier | re-root at the k-th node of the trajectory | plan again }.  After EVERY step the oracle, the reference's own LPA*
-sources (oracle/_ref; skipped where absent) and the device core built for the host (tests/cpp/lpa_emul.cpp) must agree on the
-whole state: result record, hm_ in iteration order (g, rhs, h, flags, list hashes), the priority-queue array, best_child_, the
+sources (oracle/_ref, replayed from tests/golden/reference_calls/, see tests/ref_replay.py) and the device core built for
+the host (tests/cpp/lpa_emul.cpp) must agree on the whole state: result record, hm_ in iteration order (g, rhs, h, flags, list hashes), the priority-queue array, best_child_, the
 linked points.  Two situations the reference leaves undefined end a sequence (the oracle detects them first so that the
 reference's code is never driven into them): a plan that starts on an empty priority queue, and getSubStateSpace meeting a
 stored successor that is no longer in the state space (state_space.h:160-163).  A third one was FOUND by this test (seed 21,
@@ -13,12 +13,11 @@ import numpy as np
 import pytest
 
 import oracle
-from oracle import ref
+import ref_replay as ref
+from ref_replay import recorded_reference  # noqa: F401 (autouse fixture)
 import lpa_emul
 import lpa_flow
 from test_oracle_fuzz_vs_reference import rand_case
-
-HAVE_REF = ref.available()
 
 
 def run_sequence(seed, dim, impls, rounds=4):
@@ -81,7 +80,7 @@ def run_sequence(seed, dim, impls, rounds=4):
         path = pls[0].lpa_best_child_states()[:, :dim]
         linked = [p.lpa_get_linked_nodes() for p in pls]
         for k in range(1, len(pls)):
-            assert np.array_equal(linked[0], linked[k]), (seed, dim, "linked", k)
+            assert ref.same(linked[0], linked[k]), (seed, dim, "linked", k)
         action = rng.choice(["block", "block", "clear", "subtree"])
         if action == "clear" and not dropped:
             action = "block"
@@ -126,9 +125,8 @@ def run_sequence(seed, dim, impls, rounds=4):
 
 @pytest.mark.parametrize("dim", [2, 3])
 def test_lpa_fuzz(dim):
-    impls = [(oracle.OracleMap, oracle.OraclePlanner, {}), (lpa_emul.EmuMap, lpa_emul.EmuPlanner, dict(init_cap=128, init_pred=512))]
-    if HAVE_REF:
-        impls.insert(1, (ref.RefMap, ref.RefPlanner, {}))
+    impls = [(oracle.OracleMap, oracle.OraclePlanner, {}), (ref.RefMap, ref.RefPlanner, {}),
+             (lpa_emul.EmuMap, lpa_emul.EmuPlanner, dict(init_cap=128, init_pred=512))]
     total = 0
     for seed in range(24):
         n, why = run_sequence(seed, dim, impls)

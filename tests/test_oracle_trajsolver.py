@@ -1,6 +1,6 @@
 """TrajSolver / PolySolver oracle (oracle/poly_oracle.cpp) pinned three ways (CPU only):
 (1) against the reference's OWN traj_solver.h / poly_solver.cpp / poly_traj.cpp compiled here over the stand-in Eigen
-    (oracle/_ref; skipped where /root/reference and the built library are absent) — bit for bit;
+    (oracle/_ref, replayed from tests/golden/reference_calls/, see tests/ref_replay.py) — bit for bit;
 (2) against the committed fixture tests/golden/trajsolver.npz recorded from those sources (tools/make_golden_trajsolver.py);
 (3) against the mathematics: the spline interpolates every fixed derivative, is C^(N/2-1) at interior waypoints, and no
     random perturbation of the free derivatives lowers the integral of the squared R-th derivative (the reference
@@ -12,7 +12,8 @@ import numpy as np
 import pytest
 
 import oracle
-from oracle import ref
+import ref_replay as ref
+from ref_replay import recorded_reference  # noqa: F401 (autouse fixture)
 from trajsolver_cases import ACC, JRK, SNP, VEL, cases, random_case
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "trajsolver.npz")
@@ -27,13 +28,12 @@ def poly_eval(row, t, der):
     return v
 
 
-@pytest.mark.skipif(not ref.available(), reason="needs oracle/_ref (built from /root/reference)")
 def test_oracle_equals_reference_sources():
     for name, dim, control, yaw_control, wps, dts in cases():
         a = oracle.traj_solve(dim, control, wps, dts, yaw_control)
         b = ref.traj_solve(dim, control, wps, dts, yaw_control)
         assert a.shape == b.shape == (len(wps) - 1, dim + 1, 6), name
-        assert np.array_equal(a, b), name
+        assert ref.same(a, b), name
     path = [(0, 0), (1, 0), (2, 1), (5, 1)]  # the reference's own setPath / setV(1) / allocate_time flow
     for c in (VEL, ACC, JRK):
         co, dts = ref.traj_solve_path(2, c, path, 1.0)
